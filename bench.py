@@ -7,7 +7,8 @@
 Workload (BASELINE.json configs[1]): ResNet-101 SNIPER Faster-R-CNN/R-FCN, 512x512 chips, 20 chips per
 GPU, fp32 storage with TF32 tensor-core math, synthetic COCO-shaped chips + boxes, random-init weights.
 A step = forward + backward + (N>1: one NCCL gradient all-reduce) + fused SGD-momentum update.
-`value` : chips/sec with the batch already resident in HBM (CUDA-graph replay of the step).
+`value` : chips/sec with the batch already resident in HBM (CUDA-graph replay of the step); every timed step starts
+          from the same model state, restored between steps outside the timed window.
 `e2e`   : chips/sec through Trainer.step(): pinned host batch -> H2D -> step -> D2H of the loss scalars.
 The data batches rotate through a pool larger than L2 (7 x 63 MB of input + >10 GB of activations per step),
 so no timed iteration finds its inputs in L2.
@@ -205,14 +206,53 @@ def tc_kernel_time(trainer, peak_bf16):
     return ms, flops[0], len(events), ideal_ms
 
 
-def measure(args, cfg, rank, local_rank, world, pool, dev_pool, sampler=None):
-    """Device-resident and end-to-end timing of one configuration; returns a dict (identical on every rank)."""
+DUMP_BYTES = 64 << 20
+DUMP_MAX_ELEMS = 1 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor of `arrays` as out_dir/<name>.npy, floating types as float32 and integer types as float64.
+    A tensor of more than DUMP_MAX_ELEMS elements (or one that would take the dump past DUMP_BYTES) is written as a
+    fixed sample of its flattened elements (seeded, sorted indices), the same for every run with the same arguments, so
+    that two builds can be compared output for output."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES
+    for name in sorted(arrays):
+        t = arrays[name].detach()
+        dt = torch.float32 if t.is_floating_point() else torch.float64
+        n = min(t.numel(), DUMP_MAX_ELEMS, left // (4 if dt == torch.float32 else 8))
+        if n < t.numel():
+            idx = np.unique(np.random.RandomState(0).randint(0, t.numel(), n))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.to(dt).cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes
+
+
+def measure(args, cfg, rank, local_rank, world, pool, dev_pool, sampler=None, dump_dir=None):
+    """Device-resident and end-to-end timing of one configuration; returns a dict (identical on every rank).
+    Every warm-up and timed device step starts from the model state the trainer was created with (weights, momentum,
+    BN moving statistics, restored between steps outside the timed window): the step's backward kernels accumulate
+    with float atomics, so a state carried from step to step drifts apart between runs in its last bits, and the
+    proposal selection of later steps turns that into different rois.  With the state restored, a step's inputs are the
+    same in every run with the same arguments.
+    `dump_dir`: rank 0 writes there what the last timed device step produced (its outputs and the updated weights)."""
     import torch
     import torch.distributed as dist
     from sniper_b200.trainer import Trainer
     trainer = Trainer(cfg, device="cuda:%d" % local_rank, world_size=world, use_graph=not args.no_graph)
     trainer.load(pool[0])
     trainer.capture()
+    P = trainer.net.P
+    snap = trainer._snapshot()
+    w16 = None if P.w16 is None else P.w16.clone()
+
+    def restore():
+        trainer._restore(snap)
+        if w16 is not None:
+            P.w16.copy_(w16)
 
     def barrier():
         if world > 1:
@@ -226,17 +266,21 @@ def measure(args, cfg, rank, local_rank, world, pool, dev_pool, sampler=None):
         trainer.step_device()
 
     for i in range(max(args.warmup, 3)):
+        restore()
         dev_step(i)
     if sampler is not None and rank == 0:
         sampler.start()
     barrier()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
+    ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     for i in range(args.steps):
+        restore()
+        ev[i][0].record()
         dev_step(i)
-    e1.record()
+        ev[i][1].record()
     barrier()
-    ms = e0.elapsed_time(e1)
+    ms = sum(a.elapsed_time(b) for a, b in ev)
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, dict(trainer.out, weights=trainer.net.P.w))
     # ---- end to end through the public API (host batch in, host losses out)
     for i in range(2):
         trainer.step(pool[i % len(pool)], prefetch=pool[(i + 1) % len(pool)])
@@ -543,7 +587,7 @@ def run_ours(args):
     cfg = model.Cfg()
     cfg.batch_images = args.chips
     cfg.bf16 = bool(args.bf16)
-    m = measure(args, cfg, rank, local_rank, world, pool, dev_pool, sampler)
+    m = measure(args, cfg, rank, local_rank, world, pool, dev_pool, sampler, dump_dir=args.dump_outputs)
     # ---- configs[2]'s precision (bf16 backbone + fp32 master weights) on the same N GPUs, reported as an extra block
     m3 = None
     if not args.bf16 and not args.skip_config3:
@@ -692,7 +736,12 @@ def main():
     ap.add_argument("--fp32", action="store_true", help="--config4 in fp32 storage / TF32 math")
     ap.add_argument("--skip-config4", action="store_true", help="do not append the MobileNetV2 block to the JSON line")
     ap.add_argument("--config4-multi", action="store_true", help="append the MobileNetV2 block at N > 1 too")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (outputs and updated weights, "
+                         "a fixed sample of the large ones, <= 64 MB) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.config4 or args.config5 or args.impl == "reference"):
+        ap.error("--dump-outputs applies to the ResNet-101 training bench only")
     args.iterator_leg = not args.skip_iterator
     if args.config4:
         run_config4(args)

@@ -59,13 +59,18 @@ def _ours(case):
     return _flatten(*RR.run(CW.chip_worker, cfg, RR.synth_roidb(case["seed"], **case["roidb"]), seed=1 + case["seed"]))
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree / oracle/_ref not present")
 @pytest.mark.parametrize("ci", range(len(CASES)))
 def test_matches_reference_class_executed_here(ci):
+    """Where the reference tree is not present, against the reference's outputs stored in the golden copy."""
     case = CASES[ci]
-    W = RR.load_reference_chip_worker()
-    cfg = RR.make_cfg(**case["cfg"])
-    ref = _flatten(*RR.run(W, cfg, RR.synth_roidb(case["seed"], **case["roidb"]), seed=1 + case["seed"]))
+    if HAVE_REF:
+        W = RR.load_reference_chip_worker()
+        cfg = RR.make_cfg(**case["cfg"])
+        ref = _flatten(*RR.run(W, cfg, RR.synth_roidb(case["seed"], **case["roidb"]), seed=1 + case["seed"]))
+    else:
+        gold = np.load(GOLD)
+        pre = "c%d_" % ci
+        ref = {k[len(pre):]: gold[k] for k in gold.files if k.startswith(pre)}
     ours = _ours(case)
     _same(ours, ref)
     assert ref["pos_xyxy"].shape[0] > 0

@@ -23,8 +23,11 @@ def emu():
     core = os.path.join(ROOT, "sniper_b200", "csrc", "depthwise_core.cuh")
     if not os.path.exists(OUT) or os.path.getmtime(OUT) < max(os.path.getmtime(SRC), os.path.getmtime(core)):
         os.makedirs(os.path.dirname(OUT), exist_ok=True)
-        subprocess.check_call(["nvcc", "-O2", "-std=c++17", "-Xcompiler", "-fPIC", "-shared", "-o", OUT, SRC],
+        # compiled under a private name and renamed into place: parallel test workers never load a half-written file
+        tmp = "%s.%d" % (OUT, os.getpid())
+        subprocess.check_call(["nvcc", "-O2", "-std=c++17", "-Xcompiler", "-fPIC", "-shared", "-o", tmp, SRC],
                               stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        os.replace(tmp, OUT)
     return ctypes.CDLL(OUT)
 
 

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 import oracle_lib as O
+import ref_golden as G
 from sniper_b200 import _lib, host, synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -47,7 +48,12 @@ def _config1_boxes(seed, n, W=1333, H=800):
     return b.astype(np.float32)
 
 
-@pytest.mark.skipif(O.ref_chips() is None, reason="oracle/_ref/libref_chips.so not built")
+def _ref_chips_generate(boxes, W, H, size, stride, seed):
+    """The reference's lib/chips/cchips.cpp (oracle/_ref/libref_chips.so), or its stored outputs where it is not built."""
+    run = None if O.ref_chips() is None else lambda: O.ref_chips_generate(boxes, W, H, size, stride, seed=seed)
+    return G.reference("host_cpu.chips_generate", (boxes, W, H, size, stride, seed), run)
+
+
 @pytest.mark.parametrize("scale,stride,seed", [(3.0, 58, 1), (1.667, 56, 2), (0.8, 59, 3), (0.384, 57, 4)])
 def test_chips_generate_matches_reference_cchips(scale, stride, seed):
     # config 1: one 1333x800 image, 20 GT + proposals, chip 512; reference lib/chips/cchips.cpp compiled as-is
@@ -57,7 +63,7 @@ def test_chips_generate_matches_reference_cchips(scale, stride, seed):
     W, H = int(1333 * scale), int(800 * scale)
     boxes[:, [0, 2]] = np.clip(boxes[:, [0, 2]], 0, W - 1)
     boxes[:, [1, 3]] = np.clip(boxes[:, [1, 3]], 0, H - 1)
-    ref = O.ref_chips_generate(boxes, W, H, 512, stride, seed=seed)
+    ref = _ref_chips_generate(boxes, W, H, 512, stride, seed)
     host.srand(seed)
     ours = host.chips_generate(boxes, W, H, 512, stride)
     assert ours.shape == ref.shape and ours.tobytes() == ref.tobytes()      # chip indices: bit-exact
@@ -72,8 +78,7 @@ def test_chips_empty_and_tiny_image():
     b = np.array([[10, 10, 50, 60]], np.float32)
     host.srand(1)
     c = host.chips_generate(b, 300, 200, 512, 32)      # image smaller than a chip: corner chips only
-    if O.ref_chips() is not None:
-        np.testing.assert_array_equal(c, O.ref_chips_generate(b, 300, 200, 512, 32, seed=1))
+    np.testing.assert_array_equal(c, _ref_chips_generate(b, 300, 200, 512, 32, 1))
     assert len(c) == 1
 
 
@@ -141,26 +146,32 @@ def test_gemm_launch_plan_host_logic():
 
 # ---------------------------------------------------------------------------------------------------------------
 # Pinning against the reference's OWN Cython host code (lib/nms/cpu_nms.pyx, lib/bbox/bbox.pyx), compiled from
-# /root/reference by oracle/build_ref_cython.py into oracle/_ref (4 dead tokens rewritten on the fly, see that file).
+# the reference tree by oracle/build_ref_cython.py into oracle/_ref (4 dead tokens rewritten on the fly, see that
+# file); where they are not built, their stored outputs (tests/ref_golden.py).
 # ---------------------------------------------------------------------------------------------------------------
-def _ref_cython(name):
+def _ref_cython(module, fn, *args, **kw):
+    """module.fn(*args, **kw) of the reference's Cython code built into oracle/_ref, or its stored outputs where it is
+    not built."""
     import importlib
-    ref_dir = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref")
+    ref_dir = os.path.join(ROOT, "oracle", "_ref")
     if ref_dir not in sys.path:
         sys.path.insert(0, ref_dir)
     try:
-        return importlib.import_module(name)
+        mod = importlib.import_module(module)
     except ImportError:
-        pytest.skip("oracle/_ref/%s not built (needs /root/reference and Cython at build time)" % name)
+        mod = None
+
+    def run():
+        return np.asarray(getattr(mod, fn)(*[np.copy(a) if isinstance(a, np.ndarray) else a for a in args], **kw))
+    return G.reference("host_cpu.%s.%s" % (module, fn), (args, kw), None if mod is None else run)
 
 
 @pytest.mark.parametrize("seed,n,thresh", [(0, 600, 0.7), (1, 2000, 0.5), (2, 50, 0.3)])
 def test_cpu_nms_matches_reference_cython(seed, n, thresh):
-    ref = _ref_cython("ref_cpu_nms")
     rng = np.random.RandomState(seed)
     rois = synth.rois_for_pool(rng, n, 1)
     dets = np.concatenate([rois[:, 1:], rng.permutation(n).reshape(-1, 1) / float(n)], 1).astype(np.float32)   # tie-free
-    want = [int(i) for i in ref.cpu_nms(dets.copy(), thresh)]
+    want = [int(i) for i in _ref_cython("ref_cpu_nms", "cpu_nms", dets, thresh)]
     assert host.cpu_nms(dets, thresh) == want                       # product (libsniper_b200.so, host_ops.cpp)
     assert O.cpu_nms(dets, thresh).tolist() == want                 # oracle (oracle/host.c)
     assert 0 < len(want) < n
@@ -171,12 +182,11 @@ def test_cpu_soft_nms_matches_reference_cython(method, sigma, Nt):
     """Gaussian (SNIPER's setting sigma 0.55, yml:225), linear and hard variants: same surviving rows in the same
     order; scores bit-identical for linear / hard, within 1 ulp for the Gaussian (the reference calls np.exp on a
     float32 scalar, the restatements double exp)."""
-    ref = _ref_cython("ref_cpu_nms")
     rng = np.random.RandomState(7 + method)
     n = 400
     rois = synth.rois_for_pool(rng, n, 1)
     boxes = np.concatenate([rois[:, 1:], (rng.permutation(n).reshape(-1, 1) + 1.0) / (n + 1.0)], 1).astype(np.float32)
-    want = np.array(ref.cpu_soft_nms(boxes.copy(), sigma=sigma, Nt=Nt, threshold=0.001, method=method))
+    want = _ref_cython("ref_cpu_nms", "cpu_soft_nms", boxes, sigma=sigma, Nt=Nt, threshold=0.001, method=method)
     got = host.cpu_soft_nms(boxes.copy(), sigma=sigma, Nt=Nt, threshold=0.001, method=method)
     orc = O.cpu_soft_nms(boxes.copy(), sigma=sigma, Nt=Nt, threshold=0.001, method=method)
     assert got.shape == want.shape and orc.shape == want.shape and 0 < want.shape[0] <= n
@@ -188,12 +198,11 @@ def test_cpu_soft_nms_matches_reference_cython(method, sigma, Nt):
 
 
 def test_bbox_overlaps_match_reference_cython():
-    ref = _ref_cython("ref_bbox")
     rng = np.random.RandomState(3)
     a = synth.rois_for_pool(rng, 300, 1)[:, 1:].astype(np.float64)
     b = synth.rois_for_pool(rng, 80, 1)[:, 1:].astype(np.float64)
-    want = ref.bbox_overlaps_cython(a, b)
+    want = _ref_cython("ref_bbox", "bbox_overlaps_cython", a, b)
     assert np.array_equal(host.bbox_overlaps(a, b), want) and np.array_equal(O.bbox_overlaps(a, b), want)
-    want_i = ref.ignore_overlaps_cython(a, b)
+    want_i = _ref_cython("ref_bbox", "ignore_overlaps_cython", a, b)
     assert np.array_equal(host.ignore_overlaps(a, b), want_i) and np.array_equal(O.bbox_overlaps(a, b, ignore=True), want_i)
     assert (want > 0).sum() > 100

@@ -10,6 +10,8 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+import ref_golden as G  # noqa: E402
 from sniper_b200 import iterator as IT  # noqa: E402
 
 HAVE_REF = os.path.isdir("/root/reference/lib") and os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libref_chips.so"))
@@ -34,23 +36,27 @@ def _chip_case(seed):
     return boxes, gtids, nids, classes, crop, scale
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree / oracle/_ref not present")
 @pytest.mark.parametrize("seed", range(8))
 def test_chip_ground_truth_matches_reference_anchor_worker(seed):
     """gt_boxes [100,5] bit for bit; the valid / invalid split through its only observable effect, the labels: with the
     reference's subsampling disabled (RPN_BATCH_SIZE = all anchors) the label map of the reference worker equals the
     oracle's anchor matching run on OUR (valid, invalid) sets."""
-    import run_ref_anchor_worker as RA
     import anchor_target_np as AT
     boxes, gtids, nids, classes, crop, scale = _chip_case(seed)
-    cfg = RA.make_cfg()
-    cfg.TRAIN.RPN_BATCH_SIZE = 10 ** 6          # no npr.choice subsampling: deterministic labels
-    cfg.TRAIN.RPN_FG_FRACTION = 1.0
-    W = RA.load_reference_worker()(cfg, 512)
     im_info = [512, 512, scale]
-    out = W.worker([im_info, crop.copy(), scale, nids.copy(), gtids.copy(), boxes[gtids].copy(), boxes.copy(), classes.copy()])
-    ref_label = np.asarray(out[0], np.float32).ravel()
-    ref_fgt = np.asarray(out[3], np.float64)
+
+    def run():
+        import run_ref_anchor_worker as RA
+        cfg = RA.make_cfg()
+        cfg.TRAIN.RPN_BATCH_SIZE = 10 ** 6          # no npr.choice subsampling: deterministic labels
+        cfg.TRAIN.RPN_FG_FRACTION = 1.0
+        W = RA.load_reference_worker()(cfg, 512)
+        out = W.worker([im_info, crop.copy(), scale, nids.copy(), gtids.copy(), boxes[gtids].copy(), boxes.copy(),
+                        classes.copy()])
+        return np.asarray(out[0], np.float32).ravel(), np.asarray(out[3], np.float64)
+    # where the reference is not present: its outputs stored by tests/ref_golden.py
+    ref_label, ref_fgt = G.reference("iterator_cpu.anchor_worker", (boxes, gtids, nids, classes, crop, scale),
+                                     run if HAVE_REF else None)
     valid, invalid, fgt = IT.chip_ground_truth(im_info, crop.copy(), scale, nids.copy(), gtids.copy(), boxes[gtids].copy(),
                                                boxes.copy(), classes.copy())
     assert fgt.tobytes() == ref_fgt.tobytes()

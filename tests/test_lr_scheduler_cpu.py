@@ -59,11 +59,14 @@ def test_matches_committed_golden():
         assert got == want
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree not present")
 def test_matches_reference_class_executed_here():
-    ref = _ref_class()
-    for case in CASES:
-        assert _run(lr_scheduler.WarmupMultiBatchScheduler, case) == _run(ref, case)
+    """Where the reference tree is not present, against the reference class's values stored in the golden file."""
+    if os.path.exists(REF):
+        want = [_run(_ref_class(), case) for case in CASES]
+    else:
+        want = json.load(open(GOLD))
+    for case, w in zip(CASES, want):
+        assert _run(lr_scheduler.WarmupMultiBatchScheduler, case) == w
 
 
 def test_from_config_is_the_yml_schedule():
