@@ -63,6 +63,7 @@ SIGNATURES = {
     "sniper_rpn_smooth_l1_loss": ("i", "pippiiiifpipp"),
     "sniper_softmax_ce": ("i", "pipiiifppipipp"),
     "sniper_smooth_l1_loss": ("i", "pipplifpipp"),
+    "sniper_focus_head": ("i", "pli" "ppp" "f" "p" "pppp" "p" "p"),
     "sniper_deform_im2col": ("i", "pp" "iiiiiiiiiii" "pip"),
     "sniper_deform_col2im": ("i", "ppp" "iiiiiiiiiii" "ppip"),
     "sniper_anchor_target": ("i", "ppippipp" "iiii" "pipi" "dd" "ppppp" "p"),
@@ -70,6 +71,7 @@ SIGNATURES = {
     "sniper_chip_input": ("i", "ppppiip"),
     "sniper_chip_input_hw": ("i", "ppppiiip"),
     "sniper_anchor_subsample": ("i", "pppiiiiiiup"),
+    "sniper_focus_label": ("i", "pp" "iiii" "ddd" "p" "p"),
     "sniper_chips_generate": ("i", "piiiiipi"),
     "sniper_cpu_nms": ("i", "ppidp"),
     "sniper_cpu_soft_nms": ("i", "pifffu"),

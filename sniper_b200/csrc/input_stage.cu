@@ -182,6 +182,60 @@ __global__ void __launch_bounds__(kSubTPB) anchor_subsample_kernel(float* __rest
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// AutoFocus FocusPixel labels: `gen_mask` of anchor_worker.worker (lib/data_utils/data_workers.py:165-192) on device.  A
+// box of side s = sqrt((x2-x1)*(y2-y1)) (no +1) is flagged 1 when DC_LOW < s < SMALL, -1 when SMALL <= s < DC_HIGH or
+// s <= DC_LOW, and writes nothing when s >= DC_HIGH; it covers the cells [int(x1/stride), min(ceil(x2/stride)+1, W)) x
+// (the same in y) -- one cell past the ceiling, as the reference's loop runs.  Boxes are scanned in the chip's GT order and
+// the last writer wins, so a cell keeps the flag of the last box that covers it with a non-zero flag; uncovered cells are
+// 0.  The coordinates are integers (rounded, clipped), so the product is exact in double and the correctly rounded sqrt
+// decides every threshold the way numpy does.
+// One CTA per chip: the per-box work (side, flag, cell rectangle) is done once per box into shared memory, 256 boxes at a
+// time; then each thread scans that chunk in order for the cells it owns, whose labels live in shared memory.
+constexpr int kFocusBoxes = 256;
+
+__global__ void __launch_bounds__(kFocusBoxes) focus_label_kernel(const float* __restrict__ boxes,
+                                                                  const int* __restrict__ offsets, int H, int W, int stride,
+                                                                  double dc_low, double small, double dc_high,
+                                                                  float* __restrict__ out) {
+  extern __shared__ float lab[];                    // [H*W]
+  __shared__ int4 rect[kFocusBoxes];                // cell rectangle [x1, x2) x [y1, y2); empty when the box writes nothing
+  __shared__ float flag[kFocusBoxes];
+  const int b = blockIdx.x, HW = H * W;
+  for (int c = threadIdx.x; c < HW; c += blockDim.x) lab[c] = 0.f;
+  const int k0 = offsets[b], k1 = offsets[b + 1];
+  for (int base = k0; base < k1; base += kFocusBoxes) {
+    __syncthreads();
+    const int k = base + (int)threadIdx.x;
+    if (k < k1) {
+      const double x1 = boxes[4 * (long)k], y1 = boxes[4 * (long)k + 1];
+      const double x2 = boxes[4 * (long)k + 2], y2 = boxes[4 * (long)k + 3];
+      const double area = sqrt((x2 - x1) * (y2 - y1));
+      float f = 0.f;
+      if (area > dc_low && area < small) f = 1.f;
+      else if ((area >= small && area < dc_high) || area <= dc_low) f = -1.f;
+      int4 r = make_int4((int)(x1 / stride), min((int)ceil(x2 / stride) + 1, W), (int)(y1 / stride),
+                         min((int)ceil(y2 / stride) + 1, H));
+      if (f == 0.f) r.y = r.x;                         // writes nothing
+      rect[threadIdx.x] = r;
+      flag[threadIdx.x] = f;
+    }
+    __syncthreads();
+    const int n = min(kFocusBoxes, k1 - base);
+    for (int c = threadIdx.x; c < HW; c += blockDim.x) {
+      const int y = c / W, x = c - (c / W) * W;
+      float v = lab[c];
+      for (int j = 0; j < n; ++j) {
+        const int4 r = rect[j];
+        if (x >= r.x && x < r.y && y >= r.z && y < r.w) v = flag[j];
+      }
+      lab[c] = v;
+    }
+  }
+  __syncthreads();
+  for (int c = threadIdx.x; c < HW; c += blockDim.x) out[(long)b * HW + c] = lab[c];
+}
+
 }  // namespace
 
 extern "C" {
@@ -218,6 +272,18 @@ int sniper_anchor_subsample(float* label, float* bbox_target, float* bbox_weight
   SN_CHECK(B > 0 && num_fg >= 0 && batch_size >= num_fg, "anchor_subsample: bad sizes");
   anchor_subsample_kernel<<<B, kSubTPB, 0, (cudaStream_t)stream>>>(label, bbox_target, bbox_weight, A * H * W, A, H * W,
                                                                   num_fg, batch_size, seed);
+  SN_LAUNCH_CHECK();
+  return 0;
+}
+
+// boxes: [N,4] fp32 (x1, y1, x2, y2) of every chip's GT after shift / scale / round / clip, chip-major, unfiltered;
+// offsets: int32 [B+1], chip b owns rows [offsets[b], offsets[b+1]); out: scale_label [B, H*W] in {-1, 0, 1}, fully written.
+int sniper_focus_label(const float* boxes, const int* offsets, int B, int H, int W, int stride, double dc_low,
+                       double small_thresh, double dc_high, float* out, void* stream) {
+  SN_CHECK(B > 0 && H > 0 && W > 0 && stride > 0, "focus_label: bad sizes");
+  SN_CHECK((long)H * W * 4 <= 48 * 1024, "focus_label: label map of %d x %d cells does not fit in shared memory", H, W);
+  focus_label_kernel<<<B, kFocusBoxes, (size_t)H * W * sizeof(float), (cudaStream_t)stream>>>(
+      boxes, offsets, H, W, stride, dc_low, small_thresh, dc_high, out);
   SN_LAUNCH_CHECK();
   return 0;
 }

@@ -147,6 +147,114 @@ __global__ void __launch_bounds__(256) smooth_l1_kernel(const float* __restrict_
   }
 }
 
+// AutoFocus FocusPixel head (resnet_mx_101_e2e.py:264-267, 313-315): conv_new_out (1x1, C = 256 -> 2) + SoftmaxOutput(
+// multi_output, normalization='valid', use_ignore, ignore_label=-1) + the whole backward of that layer, in one pass over
+// x3 = conv_new_3_relu [M, 256].  One warp per row: lane l holds channels [4l, 4l+4) and [128+4l, 128+4l+4) of the row
+// and of both weight rows (registers); the two logits are warp all-reductions (xor butterfly: every lane ends with the
+// same bits).  Softmax / gradient / loss arithmetic is rpn_softmax_kernel's.  dx3 = (x3 > 0) * (dz0 * W0 + dz1 * W1)
+// folds conv_new_3's ReLU backward; dW / db are per-warp register partials, summed over the block in shared memory and
+// added with one float atomic per element and block.  FP32 FMA throughout (no tensor-core contraction).
+constexpr int kFocusC = 256;
+constexpr int kFocusTPB = 256;
+
+__global__ void __launch_bounds__(kFocusTPB) focus_head_kernel(const float* __restrict__ x3, long M,
+                                                               const float* __restrict__ w, const float* __restrict__ bias,
+                                                               const float* __restrict__ label, float grad_scale,
+                                                               const int* __restrict__ valid_cnt, float* __restrict__ prob,
+                                                               float* __restrict__ dx3, float* __restrict__ dw,
+                                                               float* __restrict__ db, float* __restrict__ stats) {
+  __shared__ float red[kFocusTPB / 32][2 * kFocusC];
+  __shared__ float red_b[kFocusTPB / 32][2];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int c0 = 4 * lane, c1 = 128 + 4 * lane;
+  float w0[8], w1[8];
+  {
+    const float4 a = *reinterpret_cast<const float4*>(w + c0), b = *reinterpret_cast<const float4*>(w + c1);
+    const float4 c = *reinterpret_cast<const float4*>(w + kFocusC + c0), d = *reinterpret_cast<const float4*>(w + kFocusC + c1);
+    w0[0] = a.x; w0[1] = a.y; w0[2] = a.z; w0[3] = a.w; w0[4] = b.x; w0[5] = b.y; w0[6] = b.z; w0[7] = b.w;
+    w1[0] = c.x; w1[1] = c.y; w1[2] = c.z; w1[3] = c.w; w1[4] = d.x; w1[5] = d.y; w1[6] = d.z; w1[7] = d.w;
+  }
+  const float b0 = bias[0], b1 = bias[1];
+  const int v = *valid_cnt;
+  const float norm = grad_scale / (float)(v == 0 ? 1 : v);
+  float g0[8], g1[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) g0[j] = g1[j] = 0.f;
+  float gb0 = 0.f, gb1 = 0.f, lsum = 0.f, ncor = 0.f;
+  const long nwarps = (long)gridDim.x * (kFocusTPB / 32);
+  for (long r = (long)blockIdx.x * (kFocusTPB / 32) + wib; r < M; r += nwarps) {
+    const float* xr = x3 + r * kFocusC;
+    const float4 xa = __ldg(reinterpret_cast<const float4*>(xr + c0)), xb = __ldg(reinterpret_cast<const float4*>(xr + c1));
+    const float x[8] = {xa.x, xa.y, xa.z, xa.w, xb.x, xb.y, xb.z, xb.w};
+    float z0 = 0.f, z1 = 0.f;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      z0 = fmaf(x[j], w0[j], z0);
+      z1 = fmaf(x[j], w1[j], z1);
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+      z0 += __shfl_xor_sync(0xffffffffu, z0, off);
+      z1 += __shfl_xor_sync(0xffffffffu, z1, off);
+    }
+    z0 += b0;
+    z1 += b1;
+    const float m = fmaxf(z0, z1);
+    const float e0 = expf(z0 - m), e1 = expf(z1 - m);
+    const float inv = 1.0f / (e0 + e1);
+    const float p0 = e0 * inv, p1 = e1 * inv;
+    const int l = (int)label[r];
+    float d0 = 0.f, d1 = 0.f;
+    if (l != -1) {
+      d0 = (p0 - (l == 0 ? 1.f : 0.f)) * norm;
+      d1 = (p1 - (l == 1 ? 1.f : 0.f)) * norm;
+      lsum -= logf(fmaxf(l == 1 ? p1 : p0, 1e-14f));
+      ncor += ((p1 > p0 ? 1 : 0) == l) ? 1.f : 0.f;        // argmax_channel: the first maximum on a tie
+      gb0 += d0;
+      gb1 += d1;
+    }
+    if (lane == 0) *reinterpret_cast<float2*>(prob + 2 * r) = make_float2(p0, p1);
+    float y[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      y[j] = x[j] > 0.f ? fmaf(d1, w1[j], d0 * w0[j]) : 0.f;
+      g0[j] = fmaf(d0, x[j], g0[j]);
+      g1[j] = fmaf(d1, x[j], g1[j]);
+    }
+    float* dr = dx3 + r * kFocusC;
+    *reinterpret_cast<float4*>(dr + c0) = make_float4(y[0], y[1], y[2], y[3]);
+    *reinterpret_cast<float4*>(dr + c1) = make_float4(y[4], y[5], y[6], y[7]);
+  }
+  // block reduction of the weight / bias gradient partials, then one atomic per element
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    red[wib][c0 + j] = g0[j];
+    red[wib][c1 + j] = g0[4 + j];
+    red[wib][kFocusC + c0 + j] = g1[j];
+    red[wib][kFocusC + c1 + j] = g1[4 + j];
+  }
+  if (lane == 0) {
+    red_b[wib][0] = gb0;
+    red_b[wib][1] = gb1;
+    if (lsum != 0.f) atomicAdd(stats, lsum);
+    if (ncor != 0.f) atomicAdd(stats + 1, ncor);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < 2 * kFocusC; i += kFocusTPB) {
+    float s = 0.f;
+#pragma unroll
+    for (int k = 0; k < kFocusTPB / 32; ++k) s += red[k][i];
+    if (s != 0.f) atomicAdd(dw + i, s);
+  }
+  if (threadIdx.x < 2) {
+    float s = 0.f;
+#pragma unroll
+    for (int k = 0; k < kFocusTPB / 32; ++k) s += red_b[k][threadIdx.x];
+    if (s != 0.f) atomicAdd(db + threadIdx.x, s);
+  }
+  if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(stats + 2, (float)v);
+}
+
 int lgrid(long n) {
   long g = (n + 255) / 256;
   const long cap = (long)sn::kNumSMs * 8;
@@ -195,6 +303,25 @@ int sniper_smooth_l1_loss(const float* pred, int ld, const float* target, const 
                           float grad_scale, float* grad, int ldg, float* loss_sum, void* stream) {
   smooth_l1_kernel<<<lgrid(N * C), 256, 0, (cudaStream_t)stream>>>(pred, ld, target, weight, N, C, grad_scale, grad,
                                                                  ldg, loss_sum);
+  SN_LAUNCH_CHECK();
+  return 0;
+}
+
+// x3: [M, C] fp32 rows (C = 256, contiguous); w: [>=2, C] fp32 (rows 0 and 1 = the two classes), bias: [>=2]; label: [M]
+// in {-1, 0, 1} (-1 = ignore); valid_cnt: device int (number of labels != -1, sniper_count_valid).  Writes prob [M, 2] and
+// dx3 [M, C]; ACCUMULATES dw rows 0..1 (+= dz^T x3), db[0..1] (+= sum dz) and stats[0] += sum of -log p(label),
+// stats[1] += #correct (argmax == label), stats[2] += valid count.  Rows of w / dw beyond 1 are neither read nor written.
+int sniper_focus_head(const float* x3, long M, int C, const float* w, const float* bias, const float* label,
+                      float grad_scale, const int* valid_cnt, float* prob, float* dx3, float* dw, float* db, float* stats,
+                      void* stream) {
+  SN_CHECK(C == kFocusC, "focus_head: C must be %d", kFocusC);
+  SN_CHECK(M > 0, "focus_head: empty input");
+  SN_CHECK(((uintptr_t)x3 | (uintptr_t)w | (uintptr_t)dx3) % 16 == 0 && (uintptr_t)prob % 8 == 0,
+           "focus_head: misaligned operand");
+  long g = (M + 4 * (kFocusTPB / 32) - 1) / (4 * (kFocusTPB / 32));      // >= 4 rows per warp
+  const long cap = (long)sn::kNumSMs * 4;
+  focus_head_kernel<<<(int)(g > cap ? cap : g), kFocusTPB, 0, (cudaStream_t)stream>>>(
+      x3, M, w, bias, label, grad_scale, valid_cnt, prob, dx3, dw, db, stats);
   SN_LAUNCH_CHECK();
   return 0;
 }

@@ -40,6 +40,23 @@ def _big_enough(boxes, min_size):
     return np.where((ws >= min_size) & (hs >= min_size))[0]
 
 
+def _to_chip(b, cur_crop, im_scale, im_info):
+    """The first step of anchor_worker.worker on GT boxes (data_workers.py:210-220): shift into the chip (in place, like
+    the reference), scale, round, clip to the chip."""
+    b[:, 0] -= cur_crop[0]
+    b[:, 2] -= cur_crop[0]
+    b[:, 1] -= cur_crop[1]
+    b[:, 3] -= cur_crop[1]
+    return _clip(np.round(b * im_scale), im_info[:2])
+
+
+def chip_focus_boxes(im_info, cur_crop, im_scale, gt_boxes):
+    """The boxes AutoFocus's gen_mask rasterises (data_workers.py:220-222): EVERY GT box of the image in roidb order,
+    shifted / scaled / rounded / clipped like chip_ground_truth's, before its 10-px filter and without its cap at
+    max_n_gts.  Boxes outside the chip collapse onto its border (zero area)."""
+    return _to_chip(np.array(gt_boxes, copy=True), cur_crop, im_scale, im_info)
+
+
 def chip_ground_truth(im_info, cur_crop, im_scale, nids, gtids, gt_boxes, boxes, classes, max_n_gts=100):
     """The GT bookkeeping of anchor_worker.worker in front of the anchor matching (data_workers.py:194-281):
     shift into the chip, scale, round, clip to the chip, drop boxes under 10 px, then split the chip's GT into
@@ -48,13 +65,8 @@ def chip_ground_truth(im_info, cur_crop, im_scale, nids, gtids, gt_boxes, boxes,
     gt_boxes = np.array(gt_boxes, copy=True)
     boxes = np.asarray(boxes)
     vgt = boxes[np.intersect1d(gtids, nids)]          # fancy indexing: a copy
-    for b in (gt_boxes, vgt):
-        b[:, 0] -= cur_crop[0]
-        b[:, 2] -= cur_crop[0]
-        b[:, 1] -= cur_crop[1]
-        b[:, 3] -= cur_crop[1]
-    gt_boxes = _clip(np.round(gt_boxes * im_scale), im_info[:2])
-    vgt = _clip(np.round(vgt * im_scale), im_info[:2])
+    gt_boxes = _to_chip(gt_boxes, cur_crop, im_scale, im_info)
+    vgt = _to_chip(vgt, cur_crop, im_scale, im_info)
     ids = _big_enough(gt_boxes, 10)
     if len(ids) == 0:
         gt_boxes = np.zeros((0, 4))
@@ -82,11 +94,7 @@ class RawBatch(object):
     """Pinned host buffers of one batch (what crosses PCIe): source pixels + small per-chip arrays."""
 
     def __init__(self, B, max_gt, pixel_capacity):
-        can_pin = torch.cuda.is_available()          # host-only use (tests without a GPU): plain pageable buffers
-
-        def pin(*s, dtype):
-            t = torch.zeros(*s, dtype=dtype)
-            return t.pin_memory() if can_pin else t
+        pin = self.pin
         self.pixels = pin(pixel_capacity, dtype=torch.uint8)
         self.table = pin(B, 8, dtype=torch.int64)
         self.valid_ranges = pin(B, 2, dtype=torch.float32)
@@ -99,11 +107,23 @@ class RawBatch(object):
         self.anchor_im_info = pin(B, 3, dtype=torch.float32)
         self.used_pixels = 0
         self.seed = 0
+        # TRAIN.AUTO_FOCUS only: every chip's focus boxes (chip_focus_boxes) back to back, chip b owning rows
+        # [focus_off[b], focus_off[b+1]); focus_boxes grows with the largest batch seen
+        self.focus_boxes = None
+        self.focus_off = None
+
+    @staticmethod
+    def pin(*s, dtype):
+        t = torch.zeros(*s, dtype=dtype)
+        return t.pin_memory() if torch.cuda.is_available() else t    # host-only use (no GPU): plain pageable buffers
 
     def nbytes(self):
         small = (self.table, self.valid_ranges, self.im_info, self.gt_valid, self.ngt, self.gt_invalid, self.ninv,
                  self.gt_boxes, self.anchor_im_info)
-        return int(self.used_pixels + sum(t.numel() * t.element_size() for t in small))
+        n = int(self.used_pixels + sum(t.numel() * t.element_size() for t in small))
+        if self.focus_off is not None:
+            n += int(self.focus_off.numel() * 4 + int(self.focus_off[-1]) * 16)
+        return n
 
 
 class MNIteratorE2E(object):
@@ -123,6 +143,9 @@ class MNIteratorE2E(object):
         self.max_gt = 100
         self.data_name = ['data', 'valid_ranges', 'im_info']
         self.label_name = ['label', 'bbox_target', 'bbox_weight', 'gt_boxes']
+        self.auto_focus = bool(getattr(config.TRAIN, "AUTO_FOCUS", False))
+        if self.auto_focus:                   # MNIteratorE2E.py:28-29: the FocusPixel labels of AutoFocus training
+            self.label_name.append('scale_label')
         self.epiter = 0
         # the largest source rectangle of a chip: crop_size / (smallest scale factor) on each side, x3 channels
         self._buffers = [None] * n_buffers
@@ -232,6 +255,7 @@ class MNIteratorE2E(object):
         pix = raw.pixels.numpy()
         off = 0
         S0, S1 = self.crop_size
+        focus = []
         for k, (r, cid, (im, y1, y2, xa, xb)) in enumerate(zip(entries, cropids, rects)):
             crop = r['crops'][cid]
             im_scale = crop[1]
@@ -263,6 +287,20 @@ class MNIteratorE2E(object):
             if ni:
                 raw.gt_invalid[k, :ni] = torch.from_numpy(np.ascontiguousarray(invalid[:ni], dtype=np.float32))
             raw.gt_boxes[k] = torch.from_numpy(fgt.astype(np.float32))
+            if self.auto_focus:
+                focus.append(chip_focus_boxes(info, crop[0], im_scale, r['boxes'][gtids, :]))
+        if self.auto_focus:
+            n = sum(len(f) for f in focus)
+            if raw.focus_boxes is None or raw.focus_boxes.shape[0] < n:
+                raw.focus_boxes = raw.pin(max(int(n * 1.25), 256), 4, dtype=torch.float32)
+                raw.focus_off = raw.pin(len(focus) + 1, dtype=torch.int32)
+            o = 0
+            for k, f in enumerate(focus):
+                raw.focus_off[k] = o
+                if len(f):
+                    raw.focus_boxes[o:o + len(f)] = torch.from_numpy(np.ascontiguousarray(f, dtype=np.float32))
+                o += len(f)
+            raw.focus_off[len(focus)] = o
         raw.used_pixels = off
         raw.seed = (self.epiter * 1000003 + self.cur_i) & 0x7FFFFFFF
         return raw
@@ -347,6 +385,16 @@ class InputStage(object):
                         ngt=z(B, dtype=torch.int32), gt_invalid=z(B, max_gt, 4), ninv=z(B, dtype=torch.int32),
                         gt_boxes=z(B, max_gt, 5), anchor_im_info=z(B, 3))
         self.data = z(B, 3, crop_size, crop_size)
+        # AutoFocus training (TRAIN.AUTO_FOCUS): FocusPixel labels from the raw batch's focus boxes
+        self.auto_focus = bool(getattr(cfg.TRAIN, "AUTO_FOCUS", False))
+        if self.auto_focus:
+            T = cfg.TRAIN
+            self.focus_thresh = dict(dc_low=T.AUTO_FOCUS_DC_LOW, small_thresh=T.AUTO_FOCUS_SMALL_THRESH,
+                                     dc_high=T.AUTO_FOCUS_DC_HIGH)
+            Hf = crop_size // self.stride
+            self.focus_boxes = z(256, 4)
+            self.focus_off = z(B + 1, dtype=torch.int32)
+            self.scale_label = z(B, Hf * Hf)
 
     def run(self, raw, subsample=True):
         """H2D of the raw batch + the three kernels; returns the batch dict Trainer / SniperResNet101 consume.  Everything
@@ -370,8 +418,21 @@ class InputStage(object):
             A = len(self.scales) * len(self.ratios)
             check(lib().sniper_anchor_subsample(label.data_ptr(), bt.data_ptr(), bw.data_ptr(), self.B, A, Hf, Hf,
                                                 self.num_fg, self.rpn_batch, int(raw.seed), st))
-        return dict(data=self.data, label=label, bbox_target=bt, bbox_weight=bw, gt_boxes=self.dev["gt_boxes"],
-                    valid_ranges=self.dev["valid_ranges"], im_info=self.dev["im_info"])
+        out = dict(data=self.data, label=label, bbox_target=bt, bbox_weight=bw, gt_boxes=self.dev["gt_boxes"],
+                   valid_ranges=self.dev["valid_ranges"], im_info=self.dev["im_info"])
+        if self.auto_focus:
+            if raw.focus_off is None:
+                raise ValueError("InputStage(TRAIN.AUTO_FOCUS): the raw batch carries no focus boxes (build the iterator "
+                                 "with the same config)")
+            nb = int(raw.focus_off[-1])
+            if self.focus_boxes.shape[0] < nb:
+                self.focus_boxes = torch.zeros(int(nb * 1.25), 4, device=self.device)
+            self.focus_boxes[:nb].copy_(raw.focus_boxes[:nb], non_blocking=True)
+            self.focus_off.copy_(raw.focus_off, non_blocking=True)
+            ops.focus_label(self.focus_boxes, self.focus_off, self.B, H=Hf, W=Hf, feat_stride=self.stride,
+                            out=self.scale_label, **self.focus_thresh)
+            out["scale_label"] = self.scale_label
+        return out
 
 
 def synthetic_roidb(n_images, seed=0, width=1333, height=800, n_gt=(1, 20), n_prop=300, num_classes=81):

@@ -58,6 +58,9 @@ class Cfg:
     fuse_bn_stats = os.environ.get("SNIPER_FUSE_BN", "1") == "1"
     # run weight gradients on a second stream (see WgradScheduler); SNIPER_WGRAD_STREAM=0/1 overrides for A/B runs
     wgrad_stream = os.environ.get("SNIPER_WGRAD_STREAM", "1") == "1"
+    # AutoFocus training (TRAIN.AUTO_FOCUS, sniper_res101_e2e_autofocus.yml:106-119): the FocusPixel branch conv_new_2 ->
+    # conv_new_3 -> conv_new_out is part of the trained graph, fed by batch["scale_label"] (cls_scale_prob loss)
+    autofocus = False
 
 
 # ------------------------------------------------------------------------------------------------
@@ -533,6 +536,14 @@ class SniperResNet101:
         self.fc_new_2 = Conv(P, "fc_new_2", 1024, 1024, 1, bias=True)
         # cls_score (81) and bbox_pred (4) fused: rows [0,81) | [81,85), padded to 96
         self.fc_out = Conv(P, "cls_bbox", 1024, cfg.num_classes + 4, 1, bias=True, cout_pad=96)
+        # ---- AutoFocus branch (resnet_mx_101_e2e.py:259-267): trained in bucket 0 after the R-FCN head, fp32 after the
+        # Cast in both precisions.  conv_new_out keeps 32 rows (rows 2..31 zero, their gradients too) so that focus_map
+        # and forward_inference(autofocus=True) read the trained weights unchanged; sniper_focus_head reads rows 0..1.
+        self.af_train = bool(getattr(cfg, "autofocus", False))
+        if self.af_train:
+            self.conv_new_2 = Conv(P, "conv_new_2", 3072, 256, 3, 1, 1, 1, bias=True)
+            self.conv_new_3 = Conv(P, "conv_new_3", 256, 256, 1, bias=True)
+            self.conv_new_out = Conv(P, "conv_new_out", 256, 2, 1, bias=True, cout_pad=32, need_dgrad=False)
         P.finalize(device, lowp=bool(cfg.bf16))
         self.act_dtype = torch.bfloat16 if cfg.bf16 else torch.float32
         self._init_weights(seed, deform_offset_std)
@@ -541,7 +552,10 @@ class SniperResNet101:
         self.loss_buf = torch.zeros(8, device=device)
         self.cnt_buf = torch.zeros(2, dtype=torch.int32, device=device)
         self.step_count = 0
-        self.af = None          # AutoFocus branch (inference): enable_autofocus()
+        self.af = None          # AutoFocus branch (inference): enable_autofocus(), or the trained layers (cfg.autofocus)
+        if self.af_train:
+            self.af = [self.conv_new_2, self.conv_new_3, self.conv_new_out]
+            self.af_cnt = torch.zeros(1, dtype=torch.int32, device=device)
 
     # ---------------------------------------------------------------- AutoFocus branch (resnet_mx_101_e2e.py:259-267, 385-386)
     def enable_autofocus(self, seed=9, arg=None):
@@ -551,6 +565,9 @@ class SniperResNet101:
         layers live outside the parameter store.  arg: reference-named weights (`conv_new_2_weight` OIHW ...), else
         N(0, 0.01) like init_weight_rcnn (:468-474)."""
         from . import checkpoint as ck
+        if self.af_train:
+            raise RuntimeError("enable_autofocus(): this network trains the AutoFocus branch (Cfg.autofocus); its weights "
+                               "are parameters -- load them with load_reference")
         dev = self.device
         g = torch.Generator()
         g.manual_seed(seed)
@@ -619,6 +636,9 @@ class SniperResNet101:
         for c in (self.rpn_conv, self.rpn_head, self.conv_new_1, self.fc_new_1, self.fc_new_2, self.fc_out):
             fill(c, 0.01)
         fill(self.fc_offset, deform_offset_std and 0.001)                  # zeros in the reference (:476-477)
+        if self.af_train:                                                  # N(0, 0.01), zero biases (:468-474)
+            for c in (self.conv_new_2, self.conv_new_3, self.conv_new_out):
+                fill(c, 0.01)
         P.w.copy_(host)
         P.sync_lowp()
         pool.finalize()
@@ -639,6 +659,8 @@ class SniperResNet101:
             if not u.frozen:
                 cs += u.convs()
         cs += [self.rpn_conv, self.rpn_head, self.conv_new_1, self.fc_offset, self.fc_new_1, self.fc_new_2, self.fc_out]
+        if self.af_train:
+            cs += [self.conv_new_2, self.conv_new_3, self.conv_new_out]
         return cs
 
     # ---------------------------------------------------------------- one training step
@@ -659,8 +681,10 @@ class SniperResNet101:
 
         batch: dict of device tensors named as MNIteratorE2E provides them (MNIteratorE2E.py:175-219):
         data [B,3,512,512], label [B,A*H*W], bbox_target/bbox_weight [B,4A,H,W], gt_boxes [B,100,5],
-        valid_ranges [B,2], im_info [B,3].  Leaves parameter gradients in self.P.g and returns the outputs of
-        the reference's Group([rpn_cls_prob, rpn_bbox_loss, cls_prob, bbox_loss, label]) (:338) as a dict."""
+        valid_ranges [B,2], im_info [B,3] (+ scale_label [B,H*W] when cfg.autofocus).  Leaves parameter gradients in
+        self.P.g and returns the outputs of the reference's Group([rpn_cls_prob, rpn_bbox_loss, cls_prob, bbox_loss, label])
+        (:338) as a dict; with cfg.autofocus also cls_scale_prob (Group of :335-336), NHWC [B,H,W,2] like rpn_cls_prob (the
+        reference's is (B, 2, H*W)), and loss_buf[4:7] = (focus log-loss sum, correct count, valid count)."""
         cfg = self.cfg
         P = self.P
         A = cfg.num_anchors
@@ -670,6 +694,8 @@ class SniperResNet101:
         P.g.zero_()
         self.loss_buf.zero_()
         self.cnt_buf.zero_()
+        if self.af_train:
+            self.af_cnt.zero_()
         # weights were updated by the previous step: refresh the data-gradient operands
         if self._wt_table is None:
             jobs = [j for c in self.trainable_convs() for j in c.bwd_jobs()]
@@ -712,6 +738,16 @@ class SniperResNet101:
         rpn = self.rpn_conv.fwd(cat, relu=True)
         head = self.rpn_head.fwd(rpn)                                      # [B,H,W,128]: 4A deltas | 2A scores
         feat = self.conv_new_1.fwd(cat, relu=True)
+        if self.af_train:
+            # ---- AutoFocus branch + SoftmaxOutput('cls_scale_prob', multi_output, valid) (:259-267, 313-315): conv_new_out,
+            # the loss and its whole backward down to conv_new_3's pre-activation in one launch
+            f2 = self.conv_new_2.fwd(cat, relu=True)
+            f3 = self.conv_new_3.fwd(f2, relu=True)
+            scale_prob = torch.empty(B, Hf, Hf, 2, device=data.device)
+            df3 = torch.empty_like(f3)
+            ops.count_valid(batch["scale_label"], self.af_cnt)
+            ops.focus_head(f3, self.conv_new_out.w, self.conv_new_out.b, batch["scale_label"], cfg.grad_scale, self.af_cnt,
+                           scale_prob, df3, P.grad("conv_new_out_weight"), P.grad("conv_new_out_bias"), self.loss_buf[4:7])
         dhead = torch.zeros_like(head)
         prob = torch.empty(B, Hf, Hf, 2 * A, device=data.device)
         ops.count_valid(batch["label"], self.cnt_buf[0:1])
@@ -767,6 +803,11 @@ class SniperResNet101:
         drpn = ops.relu_bwd(rpn, self.rpn_head.bwd_data(dhead, hw))
         W(self.rpn_conv.bwd_weight, drpn, cat, sp)
         dcat = self.rpn_conv.bwd_data(drpn, hw, out=dcat, residual=dcat)
+        if self.af_train:
+            W(self.conv_new_3.bwd_weight, df3, f2, sp)
+            df2 = ops.relu_bwd(f2, self.conv_new_3.bwd_data(df3, hw))
+            W(self.conv_new_2.bwd_weight, df2, cat, sp)
+            dcat = self.conv_new_2.bwd_data(df2, hw, out=dcat, residual=dcat)
         # ---- backbone backward (stage 4, then stage 3 with the c4 half of dcat added, then stage 2)
         g, g4 = dcat[..., 1024:], dcat[..., :1024]
         if lowp:      # backward of the Cast: the backbone's activation gradients are bf16
@@ -774,6 +815,8 @@ class SniperResNet101:
         out = dict(rpn_cls_prob=prob, rpn_bbox_loss=self.loss_buf[1:2], cls_prob=cls_prob, bbox_loss=self.loss_buf[3:4],
                    label=label, rois=rois, losses=self.loss_buf, rpn_head=head, cat=cat, bbox_target=bbox_target,
                    bbox_weight=bbox_weight)
+        if self.af_train:
+            out["cls_scale_prob"] = scale_prob
         bounds = [len(self.units), n1 + n2 + n3, n1 + n2, n1]          # stage 4 | stage 3 | stage 2
         for k in range(3):
             for i in range(bounds[k] - 1, bounds[k + 1] - 1, -1):
@@ -883,7 +926,10 @@ class SniperResNet101:
     # ---------------------------------------------------------------- reference checkpoints (utils.py:45-100)
     def _named_convs(self):
         cs = [c for u in self.units for c in u.convs()]
-        return cs + [self.rpn_conv, self.rpn_head, self.conv_new_1, self.fc_offset, self.fc_new_1, self.fc_new_2, self.fc_out]
+        cs += [self.rpn_conv, self.rpn_head, self.conv_new_1, self.fc_offset, self.fc_new_1, self.fc_new_2, self.fc_out]
+        if self.af_train:
+            cs += [self.conv_new_2, self.conv_new_3, self.conv_new_out]
+        return cs
 
     def _named_bns(self):
         return [self.bn_data, self.bn0] + [b for u in self.units for b in u.bns()]

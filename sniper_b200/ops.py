@@ -656,6 +656,32 @@ def smooth_l1_loss(pred, target, weight, C, grad_scale, grad, loss_sum):
                                       grad.stride(0), _ptr(loss_sum), _stream()))
 
 
+def focus_head(x3, w, b, label, grad_scale, valid_cnt, prob, dx3, dw, db, stats):
+    """AutoFocus FocusPixel head, forward + backward in one launch.  x3: conv_new_3_relu [..., 256] fp32 rows (M rows);
+    w / b: conv_new_out weight [>=2, 256] / bias [>=2] (rows 0, 1 used); label: scale_label [M] (or [B, H*W]) in
+    {-1, 0, 1}; valid_cnt: device int32 count of labels != -1.  Writes prob [M, 2] and dx3 (the gradient of conv_new_3's
+    PRE-activation: the ReLU mask is applied); accumulates dw rows 0..1, db[0..1], and stats[0..2] += (sum of -log p,
+    correct count, valid count)."""
+    C = x3.shape[-1]
+    M = x3.numel() // C
+    assert x3.is_contiguous() and dx3.is_contiguous() and prob.is_contiguous() and w.is_contiguous()
+    assert x3.dtype == w.dtype == dx3.dtype == prob.dtype == torch.float32 and w.shape[-1] == C and label.numel() == M
+    assert prob.numel() == 2 * M and dx3.shape == x3.shape
+    check(lib().sniper_focus_head(_ptr(x3), M, C, _ptr(w), _ptr(b), _ptr(label), float(grad_scale), _ptr(valid_cnt),
+                                  _ptr(prob), _ptr(dx3), _ptr(dw), _ptr(db), _ptr(stats), _stream()))
+
+
+def focus_label(boxes, offsets, B, *, H=32, W=32, feat_stride=16, dc_low=5, small_thresh=64, dc_high=90, out=None):
+    """FocusPixel labels (gen_mask, data_workers.py:165-192): boxes [N,4] fp32 device (every chip's GT after shift /
+    scale / round / clip, chip-major, in GT order), offsets int32 [B+1] device -> scale_label [B, H*W] fp32 in {-1, 0, 1}."""
+    assert boxes.dtype == torch.float32 and boxes.is_contiguous() and offsets.dtype == torch.int32
+    if out is None:
+        out = torch.empty(B, H * W, device=offsets.device)
+    check(lib().sniper_focus_label(_ptr(boxes), _ptr(offsets), int(B), int(H), int(W), int(feat_stride), float(dc_low),
+                                   float(small_thresh), float(dc_high), _ptr(out), _stream()))
+    return out
+
+
 def deform_im2col(x, offset, *, kh=3, kw=3, stride=1, dil=1, pad=1, dgroups=4, out=None):
     """Bilinear-sampled im2col (deformable_im2col.cuh:216-263): x [N,H,W,C], offset [N,Ho,Wo,>=dg*2*kh*kw]
     -> col [N*Ho*Wo, kh*kw*C] (tap-major)."""

@@ -31,10 +31,14 @@ class NetSymbol(object):
 
     rpn_only = False        # get_symbol_rpn (resnet_mx_101_e2e.py:157-225): backbone + RPN head (+ MultiProposal at test time)
 
-    def __init__(self, cfg, is_train=True, num_classes=81, num_anchors=21, rois_per_chip=300, max_gt=100, rpn_only=False):
+    def __init__(self, cfg, is_train=True, num_classes=81, num_anchors=21, rois_per_chip=300, max_gt=100, rpn_only=False,
+                 autofocus=False):
+        """autofocus: the AutoFocus TRAINING graph (TRAIN.AUTO_FOCUS, :239-240, 259-267, 313-315, 335-336): scale_label
+        data, conv_new_2 / conv_new_3 / conv_new_out parameters, cls_scale_prob output."""
         self.cfg, self.is_train = cfg, is_train
         self.num_classes, self.num_anchors, self.rois, self.max_gt = num_classes, num_anchors, rois_per_chip, max_gt
         self.rpn_only = rpn_only
+        self.autofocus = bool(autofocus) and is_train and not rpn_only
         self._args, self._aux = [], []
         self._build()
 
@@ -83,13 +87,18 @@ class NetSymbol(object):
         self._fc("fc_new_2", 1024, 1024)
         self._fc("cls_score", K, 1024)
         self._fc("bbox_pred", 4, 1024)
+        if self.autofocus:
+            self._conv("conv_new_2", 256, 3072, 3, True)
+            self._conv("conv_new_3", 256, 256, 1, True)
+            self._conv("conv_new_out", 2, 256, 1, True)
 
     # ---- mx.sym.Symbol surface
     def data_names(self):
         if self.rpn_only:
             return ["data", "label", "bbox_target", "bbox_weight"] if self.is_train else ["data", "im_info", "im_ids"]
         if self.is_train:
-            return ["data", "im_info", "gt_boxes", "valid_ranges", "label", "bbox_target", "bbox_weight"]
+            names = ["data", "im_info", "gt_boxes", "valid_ranges", "label", "bbox_target", "bbox_weight"]
+            return names + ["scale_label"] if self.autofocus else names
         return ["data", "im_info", "im_ids", "chip_ids"]
 
     def list_arguments(self):
@@ -101,9 +110,10 @@ class NetSymbol(object):
     def list_outputs(self):
         if self.rpn_only:      # Group([rpn_cls_prob, rpn_bbox_loss]) / Group([rois, rpn_scores, im_ids]) (:214, :222)
             return ["rpn_cls_prob_output", "rpn_bbox_loss_output"] if self.is_train else ["rois_output", "rois_score", "im_ids"]
-        if self.is_train:      # mx.sym.Group order of get_symbol_rcnn (resnet_mx_101_e2e.py:336-341); metric.py reads it by position
-            return ["rpn_cls_prob_output", "rpn_bbox_loss_output", "cls_prob_reshape_output", "bbox_loss_reshape_output",
-                    "blockgrad0_output"]
+        if self.is_train:      # mx.sym.Group order of get_symbol_rcnn (resnet_mx_101_e2e.py:335-338); metric.py reads it by position
+            names = ["rpn_cls_prob_output", "rpn_bbox_loss_output", "cls_prob_reshape_output", "bbox_loss_reshape_output",
+                     "blockgrad0_output"]
+            return names[:2] + ["cls_scale_prob_output"] + names[2:] if self.autofocus else names
         # test-time group (:386-389): rois, cls_prob, bbox_pred and the three pass-through inputs
         return ["rois_output", "cls_prob_reshape_output", "bbox_pred_reshape_output", "im_ids", "im_info", "chip_ids"]
 
@@ -114,7 +124,8 @@ class NetSymbol(object):
         A, K, R = self.num_anchors, self.num_classes, self.rois
         dflt = {"data": data_shapes["data"], "im_info": (B, 3), "im_ids": (B,), "chip_ids": (B,),
                 "gt_boxes": (B, self.max_gt, 5), "valid_ranges": (B, 2),
-                "label": (B, A * H * W), "bbox_target": (B, 4 * A, H, W), "bbox_weight": (B, 4 * A, H, W)}
+                "label": (B, A * H * W), "bbox_target": (B, 4 * A, H, W), "bbox_weight": (B, 4 * A, H, W),
+                "scale_label": (B, H * W)}
         arg = [tuple(data_shapes.get(n, dflt[n])) for n in self.data_names()] + [s for _, s in self._args]
         if self.rpn_only:
             out = [(B, 2, A * H, W), (B, 4 * A, H, W)] if self.is_train else [(B * R, 5), (B * R,), (B,)]
@@ -122,6 +133,8 @@ class NetSymbol(object):
         if self.is_train:
             # the last head is BlockGrad(label_reshape): Reshape(label, (-1,)) (resnet_mx_101_e2e.py:281,334) -> (B*R,)
             out = [(B, 2, A * H, W), (B, 4 * A, H, W), (B, R, K), (B, R, 4), (B * R,)]
+            if self.autofocus:          # cls_scale_prob over conv_new_out_reshape (0, 2, -1) (:266, 313-315)
+                out.insert(2, (B, 2, H * W))
         else:
             out = [(B * R, 5), (B, R, K), (B, R, 4), (B,), (B, 3), (B,)]
         return arg, out, [s for _, s in self._aux]
@@ -132,6 +145,7 @@ class NetSymbol(object):
         c = model.Cfg()
         c.batch_images = batch_images
         c.bf16 = bool(bf16)
+        c.autofocus = self.autofocus
         for k, v in cfg_overrides.items():
             setattr(c, k, v)
         return model.SniperResNet101(c, device=device, seed=seed)
@@ -247,8 +261,14 @@ def recognise_graph(sym):
     theirs_aux = {n: tuple(s) for n, s in zip(sym.list_auxiliary_states(), auxs)}
     mine = {n: tuple(s) for n, s in ours._args}
     mine_aux = {n: tuple(s) for n, s in ours._aux}
-    # the AutoFocus branch (conv_new_2/3/out) is optional: model.enable_autofocus()
+    # the AutoFocus branch (conv_new_2/3/out): trained when the graph is a training graph with the scale_label loss
+    # (TRAIN.AUTO_FOCUS), else the inference branch of model.enable_autofocus()
     af = {k for k in theirs if k.startswith(("conv_new_2_", "conv_new_3_", "conv_new_out_"))}
+    af_train = bool(af) and is_train and "cls_scale_prob" in nodes
+    if af_train:
+        ours = NetSymbol(None, is_train=True, num_classes=K, num_anchors=A, autofocus=True)
+        mine = {n: tuple(s) for n, s in ours._args}
+        af = set()
     diff = sorted((set(theirs) - af) ^ set(mine)) + sorted(set(theirs_aux) ^ set(mine_aux))
     diff += sorted(k for k in mine if k in theirs and theirs[k] != mine[k])
     if diff:
@@ -256,7 +276,9 @@ def recognise_graph(sym):
                                   "graph differs in %d parameters, e.g. %s" % (len(diff), ", ".join(diff[:6])))
     if mnv2 and not is_train:
         raise NotImplementedError("MobileNetV2: only the training graph is executable")
-    info = dict(batch_images=B, num_anchors=A, num_classes=K, bf16=fp16, is_train=is_train, autofocus=bool(af))
+    info = dict(batch_images=B, num_anchors=A, num_classes=K, bf16=fp16, is_train=is_train, autofocus=bool(af) or af_train)
+    if af_train:                              # the executor trains the FocusPixel branch (Cfg.autofocus)
+        info["autofocus_train"] = True
     if mnv2:
         info["network"] = "mobilenetv2"
     if rpn_only:
@@ -273,12 +295,15 @@ def bind_graph(sym, device="cuda:0", **overrides):
     info = recognise_graph(sym)
     cls = MobileNetSymbol if info.get("network") == "mobilenetv2" else NetSymbol
     ours = cls(None, is_train=info["is_train"], num_classes=info["num_classes"], num_anchors=info["num_anchors"])
+    if info.get("autofocus_train"):               # the FocusPixel branch is trained: Cfg.autofocus (not enable_autofocus)
+        ours = NetSymbol(None, is_train=True, num_classes=info["num_classes"], num_anchors=info["num_anchors"],
+                         autofocus=True)
     # (an RPN-only test graph binds to the full network object: its executor is `forward_rpn`)
     kw = dict(batch_images=info["batch_images"], bf16=info["bf16"], num_classes=info["num_classes"],
               num_anchors=info["num_anchors"])
     kw.update(overrides)
     net = ours.bind(device, **kw)
-    if info["autofocus"]:
+    if info["autofocus"] and not info.get("autofocus_train"):
         net.enable_autofocus()
     return net
 
@@ -362,7 +387,8 @@ class resnet_mx_101_e2e(Symbol):
         num_classes = getattr(getattr(cfg, "dataset", None), "NUM_CLASSES", 81)
         net = getattr(cfg, "network", None)
         num_anchors = getattr(net, "NUM_ANCHORS", 21) if net is not None else 21
-        self.sym = NetSymbol(cfg, is_train=is_train, num_classes=num_classes, num_anchors=num_anchors)
+        autofocus = bool(getattr(getattr(cfg, "TRAIN", None), "AUTO_FOCUS", False))
+        self.sym = NetSymbol(cfg, is_train=is_train, num_classes=num_classes, num_anchors=num_anchors, autofocus=autofocus)
         return self.sym
 
     get_symbol = get_symbol_rcnn
@@ -398,6 +424,10 @@ class resnet_mx_101_e2e(Symbol):
         for n in ('rpn_conv_3x3', 'rpn_cls_score', 'rpn_bbox_pred', 'conv_new_1'):
             arg_params[n + '_weight'] = normal(n + '_weight')
             arg_params[n + '_bias'] = zeros(n + '_bias')
+        if getattr(self.sym, "autofocus", False):              # TRAIN.AUTO_FOCUS (:468-474)
+            for n in ('conv_new_2', 'conv_new_3', 'conv_new_out'):
+                arg_params[n + '_weight'] = normal(n + '_weight')
+                arg_params[n + '_bias'] = zeros(n + '_bias')
         arg_params['offset_weight'] = zeros('offset_weight')
         arg_params['offset_bias'] = zeros('offset_bias')
         for n in ('fc_new_1', 'fc_new_2', 'cls_score', 'bbox_pred'):

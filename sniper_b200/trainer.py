@@ -6,7 +6,7 @@ next batch: `step(batch, prefetch=next_batch)`, as MNIteratorE2E's prefetch thre
 forward+backward, ONE NCCL all-reduce over the flat gradient bucket (replaces the per-key kvstore
 push/pull, model.py:126-136 / comm.h:433-553; sum without 1/N as rescale_grad=1.0, utils.py:30,37), one
 CUDA-graph replay of the fused SGD-momentum update, D2H of the four loss scalars (what the reference's
-metrics read with asnumpy(), lib/train_utils/metric.py:109-125).
+metrics read with asnumpy(), lib/train_utils/metric.py:109-125; with AutoFocus training also its two metrics, :50-94).
 """
 import torch
 
@@ -197,6 +197,19 @@ class Trainer:
             self.net.update()
         return self.out
 
+    def _losses(self):
+        """The host loss scalars of the step just run.  A network that trains the AutoFocus branch (Cfg.autofocus) adds the
+        two AutoFocus metrics of lib/train_utils/metric.py:50-94 for this batch: AutoFocusLogLoss (mean -log p(label)
+        over the FocusPixel labels != -1) and AutoFocusAcc (argmax == label over the same); nan without a valid label."""
+        h = self.loss_host
+        res = {"rpn_cls_loss": float(h[0]), "rpn_bbox_loss": float(h[1]), "rcnn_cls_loss": float(h[2]),
+               "rcnn_bbox_loss": float(h[3]), "lr": self.lr}
+        if getattr(self.net, "af_train", False):
+            n = float(h[6])
+            res["autofocus_logloss"] = float(h[4]) / n if n > 0 else float("nan")
+            res["autofocus_acc"] = float(h[5]) / n if n > 0 else float("nan")
+        return res
+
     # ---- public end-to-end step from the iterator's raw batch (uint8 source rectangles + chip tables)
     def step_raw(self, raw, input_stage, lr=None):
         """One training step on a `iterator.RawBatch`: H2D of the raw bytes, GPU input stage (resize / mean / flip,
@@ -211,8 +224,7 @@ class Trainer:
         out = self.step_device(lr)
         self.loss_host.copy_(out["losses"], non_blocking=True)
         torch.cuda.current_stream().synchronize()
-        return {"rpn_cls_loss": float(self.loss_host[0]), "rpn_bbox_loss": float(self.loss_host[1]),
-                "rcnn_cls_loss": float(self.loss_host[2]), "rcnn_bbox_loss": float(self.loss_host[3]), "lr": self.lr}
+        return self._losses()
 
     # ---- public end-to-end step: host batch in, host losses out
     def step(self, host_batch, prefetch=None, lr=None):
@@ -227,5 +239,4 @@ class Trainer:
         out = self.step_device(lr)
         self.loss_host.copy_(out["losses"], non_blocking=True)
         torch.cuda.current_stream().synchronize()
-        return {"rpn_cls_loss": float(self.loss_host[0]), "rpn_bbox_loss": float(self.loss_host[1]),
-                "rcnn_cls_loss": float(self.loss_host[2]), "rcnn_bbox_loss": float(self.loss_host[3]), "lr": self.lr}
+        return self._losses()

@@ -54,6 +54,7 @@ DOC = {
     "sniper_rpn_smooth_l1_loss": "weight * smooth_l1(pred - target) + MakeLoss gradient for the RPN (mshadow_op.h:642-678; resnet_mx_101_e2e.py:330-334).",
     "sniper_softmax_ce": "SoftmaxOutput(normalization=valid, use_ignore) flat form (softmax_output-inl.h:207-263).",
     "sniper_smooth_l1_loss": "weight * smooth_l1(pred - target) + MakeLoss gradient (resnet_mx_101_e2e.py:318-319).",
+    "sniper_focus_head": "AutoFocus FocusPixel head: conv_new_out (1x1, 256 -> 2) + SoftmaxOutput(multi_output, normalization=valid, use_ignore, ignore_label=-1) (resnet_mx_101_e2e.py:264-267, 313-315; softmax_output-inl.h:162-206, 225-257) + its whole backward (dx3 with conv_new_3's ReLU mask, dW +=, db +=) in one pass; log-loss sum, correct count and valid count of AutoFocusLogLoss / AutoFocusAcc (lib/train_utils/metric.py:50-94) accumulated on the device.",
     "sniper_deform_im2col": "deformable_im2col (contrib/nn/deformable_im2col.cuh:216-263), NHWC, whole batch.",
     "sniper_deform_col2im": "deformable_col2im + deformable_col2im_coord (contrib/nn/deformable_im2col.cuh:317-360, 419-480).",
     "sniper_anchor_target": "RPN anchor matching of anchor_worker.worker (lib/data_utils/data_workers.py:164-371) on device.",
@@ -61,6 +62,7 @@ DOC = {
     "sniper_chip_input": "GPU input stage: im_worker.worker (lib/data_utils/data_workers.py:80-121) -- flip, cv2-style 8-bit bilinear resize by the chip scale, zero padding to crop_size, BGR->RGB minus PIXEL_MEANS -- from uint8 source rectangles to the fp32 NCHW `data` tensor of MNIteratorE2E (lib/iterators/MNIteratorE2E.py:194-199).",
     "sniper_chip_input_hw": "The same with a rectangular canvas: im_worker.worker_autofocus (lib/data_utils/data_workers.py:51-78) + the batch padding of MNIteratorTestAutoFocus._get_batch (lib/iterators/MNIteratorTestAutoFocus.py:36-78).",
     "sniper_anchor_subsample": "The npr.choice subsampling of anchor_worker.worker (data_workers.py:326-338) on device: <= num_fg positives, <= batch_size - #positives negatives per chip, the rest -> -1 (counter-based hash instead of numpy's RNG).",
+    "sniper_focus_label": "FocusPixel labels of AutoFocus training: gen_mask of anchor_worker.worker (lib/data_utils/data_workers.py:165-192, called at :220-222) on device, one thread per label cell, boxes in GT order (last writer wins) -> scale_label [B, H*W] of MNIteratorE2E (lib/iterators/MNIteratorE2E.py:182-197).",
     "sniper_chips_generate": "chips::cgenerate (lib/chips/cchips.cpp:54-177): host-side chip sampling, same rand() stream.",
     "sniper_cpu_nms": "cpu_nms (lib/nms/cpu_nms.pyx:112-163), host.",
     "sniper_cpu_soft_nms": "cpu_soft_nms (lib/nms/cpu_nms.pyx:17-110), host, in place.",
